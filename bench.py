@@ -1,14 +1,14 @@
 #!/usr/bin/env python3
 """bench.py -- k-mer insert+lookup throughput of the B200 engine on BASELINE.json config 2.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): 10 M synthetic 150 bp SE reads from a 100 Mbp random genome, 0.5 % substitutions, `-gs 100`
 k-mer lengths (prefix 12, p17/s20/b24), original order.  The job is ONE stream of reads (fqsqueezer_b200/synth.py: job_chunk) cut
 into reads_blocks exactly where the reference cuts the corresponding FASTQ (16 MiB slabs, reads_block.h:121-169 -> 196 blocks) and
 every block into calc_no_synchronizations(g) + 1 sync segments (application.h:85-92); every segment is one fqsk_segment + fqsk_sync.
 
-A STEP is 1/K of that job: step j covers blocks [196 j / K, 196 (j + 1) / K), so any --steps spans both regimes of the job -- the
+A STEP is 1/K of that job: step j covers blocks [196 j / K, 196 (j + 1) / K) (1 <= K <= 196), so any --steps spans both regimes of the job -- the
 EARLY one (blocks 0..99: 100 - g sync segments per block, latency bound) and the STEADY one (blocks 100+: one 51 k-read segment per
 block) -- which are also timed and reported separately (`regimes`).  The W warm-up steps run the first W steps of the job on a
 throw-away engine (same work, untimed).
@@ -19,6 +19,11 @@ e2e    : the same steps through the host-buffer C-ABI calls (fqsk_submit_ctx / f
 parity_check : device-side checksums (fqsk_recs_checksum) of every sync segment of the first blocks of the timed job against the
          REAL reference's records for the same reads (tests/golden/bench_config2_ref_checksums.npz, produced once by
          oracle/make_bench_golden.py from the tapped fqs-1.1 at -t 1).
+--dump-outputs DIR : after the timed steps, what fqsk_segment_device handed its caller in every sync segment of the LAST timed step, as
+         float64 .npy files: the number of records and their device checksum per segment, and a fixed, seeded sample of the per-base
+         records (at most 2^19 + one per segment, under 40 MB in all).  The inputs depend on nothing but the arguments, so two builds
+         can be compared output for output.  Taking the sample waits for every segment of that step inside the timed region, so the
+         line then carries "timing_comparable": false.  Not with --impl reference or N > 1.
 N > 1  : ONE job over N GPUs, tables hash-sharded by the reference's owner keys (reference `-t N` semantics; scaling "strong");
          `--replicas` runs N independent engines instead (weak scaling, no exchange).
 roofline / cpu_baseline / compress_e2e: see DESIGN.md section 7.
@@ -110,6 +115,58 @@ def codes_to_slab(codes):
     off = (np.arange(n, dtype=np.uint64) * np.uint64(L + 1))
     ln = np.full(n, L, np.uint32)
     return slab.reshape(-1), off, ln
+
+
+DUMP_SAMPLE = 1 << 19               # records of the last timed step kept by --dump-outputs (8 float64 columns each: 32 MiB)
+DUMP_SEED = 7
+REC_FIELDS = ["pos", "c0", "c1", "c2", "c3", "cor_pos", "level", "rough"]      # fqsk_base_rec (include/fqsk.h) without its padding
+
+
+class _DeviceBytes:
+    """A device buffer owned by the engine, handed to torch without a copy (__cuda_array_interface__)."""
+
+    def __init__(self, ptr, nbytes):
+        self.__cuda_array_interface__ = {"shape": (nbytes,), "typestr": "|u1", "data": (ptr, False), "version": 3}
+
+
+class LastStepOutputs:
+    """--dump-outputs: per sync segment of the last timed step, the records fqsk_segment_device leaves in device memory for its caller --
+    their number, the device checksum of all of them (fqsk_recs_checksum) and a seeded sample of them; the sample takes a share of
+    DUMP_SAMPLE proportional to the segment's reads, at positions drawn from a generator seeded with the segment's ordinal."""
+
+    def __init__(self, reads_in_step, dev):
+        self.reads_in_step, self.dev = reads_in_step, dev
+        self.n_recs, self.sums, self.index, self.rows = [], [], [], []
+        self.first = 0                  # position of the current segment's first record in the step's record stream
+
+    def capture(self, eng, n_reads):
+        import torch
+        from fqsqueezer_b200 import engine as E
+        cs, n = eng.recs_checksum()     # settles the segment and waits for the engine's stream
+        ptr, n_dev = eng.device_recs()
+        assert n_dev == n, (n_dev, n)
+        m = min(n, -(-DUMP_SAMPLE * n_reads // self.reads_in_step))
+        idx = np.unique(np.random.default_rng([DUMP_SEED, len(self.n_recs)]).integers(0, n, m)) if m else np.zeros(0, np.int64)
+        if len(idx):
+            rb = E.REC_DTYPE.itemsize
+            recs = torch.as_tensor(_DeviceBytes(ptr, n * rb), device=self.dev).view(torch.int32).view(n, rb // 4)
+            w = recs[torch.from_numpy(idx).to(self.dev)].cpu().numpy().view(np.uint32)      # .cpu() waits: the next segment reuses the buffer
+            self.rows.append(np.stack([w[:, 0], w[:, 1], w[:, 2], w[:, 3], w[:, 4], w[:, 5], w[:, 6] & 0xFF, (w[:, 6] >> 8) & 0xFF], axis=1).astype(np.float64))
+            self.index.append((self.first + idx).astype(np.float64))
+        self.n_recs.append(n)
+        self.sums.append((cs >> 32, cs & 0xFFFFFFFF))
+        self.first += n
+
+    def write(self, out_dir):
+        os.makedirs(out_dir, exist_ok=True)
+        arrays = {"segment_n_records": np.array(self.n_recs, np.float64),
+                  "segment_checksum_hi_lo": np.array(self.sums, np.float64).reshape(-1, 2),
+                  "records_sample": np.concatenate(self.rows) if self.rows else np.zeros((0, len(REC_FIELDS)), np.float64),
+                  "records_sample_index": np.concatenate(self.index) if self.index else np.zeros(0, np.float64)}
+        for name, a in arrays.items():
+            np.save(os.path.join(out_dir, name + ".npy"), a)
+        return {"dir": out_dir, "segments": len(self.n_recs), "records": int(self.first), "sampled": len(arrays["records_sample_index"]),
+                "records_sample_columns": REC_FIELDS, "bytes": sum(a.nbytes for a in arrays.values())}
 
 
 class ClockSampler(threading.Thread):
@@ -379,10 +436,14 @@ def main():
     ap.add_argument("--max-blocks", type=int, default=0, help="debug: stop the job after this many blocks")
     ap.add_argument("--trace-blocks", type=int, default=0, help="print per-block phase ms every N blocks to stderr")
     ap.add_argument("--profile-block", type=int, default=-1, help="cudaProfilerStart/Stop around this block (for ncu --profile-from-start off)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the records of the last timed step (per-segment counts and checksums, "
+                    "a seeded sample of the records) as DIR/<name>.npy; one engine only")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs: the records come from the engine's timed path; --impl reference has none")
         return reference_arm(args)
 
     import torch
@@ -409,7 +470,11 @@ def main():
         blocks = blocks[: args.max_blocks]
     NB = len(blocks)
     K = args.steps
-    step_of_block = [min(K - 1, g * K // NB) for g in range(NB)] if K <= NB else list(range(NB))
+    if not 1 <= K <= NB:
+        raise SystemExit(f"--steps {K}: a step is 1/K of the job's {NB} reads_blocks, so 1 <= --steps <= {NB}")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs: one engine only (no --gpus > 1)")
+    step_of_block = [g * K // NB for g in range(NB)]
     # warm-up: W steps of the job on a throw-away engine -- and, unless --short-warmup, the rest of the job behind them: a fresh box needs
     # seconds, not steps, until its host side runs at speed (the first bench run on a fresh box measured 3x the launch work of the second,
     # profiles/r02_bench_first_run_on_a_fresh_box.json), and the later blocks use launch paths (51 000-read segments) the first W steps never touch
@@ -455,7 +520,7 @@ def main():
         d_blocks.append((lo, torch.from_numpy(synth.codes_to_ascii(codes).reshape(-1)).to(dev)))
     torch.cuda.synchronize()
 
-    def run_block_device(g, e):
+    def run_block_device(g, e, capture=None):
         e.block_start()
         lo, t = d_blocks[g]
         base = t.data_ptr()
@@ -463,6 +528,8 @@ def main():
         for k, (a, bb) in enumerate(segs):
             n = bb - a
             e.segment_device(base + (a - lo) * L, n * L, d_off.data_ptr(), d_len.data_ptr(), n, want_n_recs=False)
+            if capture is not None:
+                capture(e, n)
             if k + 1 < len(segs):      # the worker loop knows its next segment (application.cpp:617-662): its read-only preparation runs ahead
                 a2, b2 = segs[k + 1]
                 e.announce_device(base + (a2 - lo) * L, (b2 - a2) * L, d_off.data_ptr(), d_len.data_ptr(), b2 - a2)
@@ -485,6 +552,9 @@ def main():
     prev_prof, t_prev = eng.profile(), time.time()
     regime_ms = {"early": 0.0, "steady": 0.0}
     seg_early = 0
+    last_step = None
+    if args.dump_outputs:
+        last_step = LastStepOutputs(sum(sched[g][-1][1] - sched[g][0][0] for g in range(NB) if step_of_block[g] == K - 1), dev)
 
     def run_range(g0, g1, key):
         nonlocal prev_prof, t_prev
@@ -494,7 +564,7 @@ def main():
         for g in range(g0, g1):
             if g == args.profile_block:
                 torch.cuda.cudart().cudaProfilerStart()
-            run_block_device(g, eng)
+            run_block_device(g, eng, last_step.capture if last_step is not None and step_of_block[g] == K - 1 else None)
             if g == args.profile_block:
                 torch.cuda.cudart().cudaProfilerStop()
             if args.trace_blocks and (g % args.trace_blocks == 0 or g == NB - 1):
@@ -532,6 +602,7 @@ def main():
         dist.all_reduce(lt)
         launches = int(lt.item())
     eng.close()
+    dumped = last_step.write(args.dump_outputs) if last_step is not None else None
 
     # ---------------- phase shares: the same pass again with CUDA-event brackets around the internal phases ----------------
     phases = None
@@ -730,6 +801,11 @@ def main():
                     "warmup_blocks": len(warm_blocks), "warmup_note": "untimed, on a throw-away engine with its own tables: the W warm-up steps" + ("" if args.short_warmup else " and the rest of the job behind them"), "note": "table construction (fqsk_create) lies outside the timed region, as the reference's does in its arm"},
             "regimes": regimes, "roofline": roof, "parity_check": parity, "cpu_baseline": cpu, "e2e": e2e, "compress_e2e": compress, "gpu_launches": int(launches),
             "clocks": sampler.summary(), "wall_ms_per_step": wall_ms / K}
+    if dumped is not None:      # the capture sits inside the timed region: this line's timings are not those of a plain run
+        line["dump_outputs"] = dumped
+        line["timing_comparable"] = False
+        line["timing_note"] = ("--dump-outputs: every sync segment of the last step waited for a device checksum and a sampled copy of its records inside the "
+                               "timed region; value, ms_per_step, regimes, job and gpu_launches are not comparable with a run without it")
     print(json.dumps(line))
     if dist is not None:
         dist.destroy_process_group()

@@ -9,8 +9,8 @@ Result (round 1, block 0, 51 000 reads, -gs 100):
 i.e. the trajectory (registers, repairs, s-/b-mer pushes) of an early block does not depend on the intra-block syncs at all; what does
 is the p-mer level (the 2-bit array has no thread-local twin, so only a sync makes a p-mer visible) and a handful of s-/b-level counts.
 This is the evidence behind DESIGN.md's round-2 plan (block-level pass + versioned fix-up).   Run: python tests/probe_block_visibility.py (~6 min)"""
-import sys, time, numpy as np
-sys.path.insert(0,'/root/repo')
+import os, sys, time, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from fqsqueezer_b200 import synth, schedule as S, engine as E
 from oracle import oracle as O
 import bench

@@ -10,8 +10,8 @@ Result (round 1):
 i.e. with populated tables the cross-segment dependence is carried by COUNT VALUES (a b-mer seen once more), rarely by the trajectory
 (cor_pos 1.25 %, pushes 0.5 %) -- at ten times the real density.  At config-2 density expect about a tenth of it: the versioned
 counts of DESIGN.md's round-2 plan are needed for ~2 % of the records of a late early block, the re-walk set stays small."""
-import sys, time, numpy as np
-sys.path.insert(0,'/root/repo')
+import os, sys, time, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from fqsqueezer_b200 import synth, schedule as S, engine as E
 from oracle import oracle as O
 import bench

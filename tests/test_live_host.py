@@ -6,7 +6,8 @@ CPU leg : $FQSK_LIB = a mock built from the oracle (tests/mock_fqsk.cpp).  Check
 GPU leg : $FQSK_LIB = fqsqueezer_b200/libfqsk.so.  The whole thing: reads_block slabs -> fqsk_segment / fqsk_sync on the B200 ->
           the reference's context model and range coders.
 Both: the .fqs is byte-identical to the unmodified `fqs-1.1 -t 1` and the unmodified binary decodes it back to the input.
-The binaries are built from /root/reference by __graft_entry__.build() and travel to the GPU box (host/_bin, oracle/_ref)."""
+The binaries (host/_bin, oracle/_ref) are built from the reference's sources, which the repository does not contain.  Where they are
+absent, the GPU legs check the engine half of the same run instead (_engine_half)."""
 import os
 import subprocess
 import tempfile
@@ -14,13 +15,65 @@ import tempfile
 import numpy as np
 import pytest
 
+from fqsqueezer_b200 import engine as E
+from fqsqueezer_b200 import schedule as S
 from fqsqueezer_b200 import synth
 from oracle import oracle as O
+from tests import helpers as H
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIVE_BIN = os.path.join(ROOT, "host", "_bin", "fqs-1.1-fqsk")
 REAL_LIB = os.path.join(ROOT, "fqsqueezer_b200", "libfqsk.so")
-needs_bins = pytest.mark.skipif(not (os.path.exists(O.REF_BIN) and os.path.exists(LIVE_BIN)), reason="host/_bin or oracle/_ref not built")
+HAVE_BINS = os.path.exists(O.REF_BIN) and os.path.exists(LIVE_BIN)
+needs_bins = pytest.mark.skipif(not HAVE_BINS, reason="host/_bin or oracle/_ref not built")
+
+
+def _fastq_records(path):
+    slab = np.fromfile(path, np.uint8)
+    _, _, roff, rsz = S.parse_fastq(slab)
+    return [slab[int(a):int(a) + int(n)] for a, n in zip(roff, rsz)]
+
+
+def _engine_half(files, gs, layout=("-s", "-om", "o"), submit=False):
+    """The engine half of a drop-in run, for a checkout without the binaries: the reads of `files` in the order the drop-in hands them to
+    libfqsk.so (pairs interleaved; in sorted order (-om s) ordered by the comparator of CSortedFASTQFile::sort_reads, of mate 1 when
+    paired), through the C-ABI on the GPU -- fqsk_submit / fqsk_collect when `submit`, else fqsk_segment / fqsk_sync -- against the CPU
+    oracle on the same schedule (pinned to the tapped reference by test_golden_oracle): records, pair decisions, sorted-prefix flags and
+    difs and every table, bit-exact."""
+    paired, srt = layout[0] == "-p", layout[-1] == "s"
+    recs = [_fastq_records(f) for f in files]
+    recs = [r for pair in zip(*recs) for r in pair] if paired else recs[0]
+    step = 2 if paired else 1
+    if srt:
+        first = np.concatenate(recs[0::step])
+        off, ln, _, _ = S.parse_fastq(first)
+        order = np.argsort(O.sort_ranks(first, off, ln), kind="stable")
+        recs = [r for i in order for r in recs[step * i:step * i + step]]
+    slab = np.concatenate(recs)
+    mode = (2 if paired else 0) + (1 if srt else 0)
+    pref, p, s, b = E.kmer_params(gs)
+    e = E.KmerEngine(p, s, b, pref, mode=mode)
+    o = O.OracleEngine(p, s, b, pref, mode=mode)
+    if submit:
+        assert not srt
+        got = H.run_async(e, slab, paired=paired)
+        got = (got[0], got[2]) if paired else got[:1]
+        want = H.run_pe(o, slab) if paired else (H.run_se(o, slab),)
+    else:
+        run = {0: lambda x, g: (H.run_se(x, slab),), 1: lambda x, g: H.run_sorted(x, slab, g), 2: lambda x, g: H.run_pe(x, slab, g),
+               3: lambda x, g: H.run_pe_sorted(x, slab, g)}[mode]
+        got, want = run(e, True), run(o, False)
+    H.assert_recs_equal(got[0], want[0][want[0]["pos"] < 0xFFFFFFF0])
+    assert len(got[0]) > 1000
+    for i in range(1, len(want)):
+        assert np.array_equal(got[i], want[i]), i
+    for which in range(4 if paired else 3):
+        kg, vg = e.dump(which)
+        ko, vo = o.dump(which)
+        assert np.array_equal(kg, ko) and np.array_equal(vg, vo), which
+    assert e.stats()["kernel_launches"] > 0
+    e.close(); o.close()
+
 
 # (gs, genome, reads, read length, seed, N fraction, duplicate fraction)
 CASES = [(1, 6000, 4000, 100, 31, 0.002, 0.01), (100, 40000, 3000, 150, 32, 0.0, 0.0)]
@@ -85,6 +138,14 @@ PAIRED = [(1, 5000, 1200, 80, 71), (100, 50000, 4000, 150, 72)]
 PAIRED_SORTED = [(1, 5000, 1500, 80, 73), (100, 50000, 4000, 150, 74)]
 
 
+def _engine_half_of(case, layout):
+    """_engine_half on the input _run_sorted / _run_paired generate for `case`."""
+    gs, G, n, L, seed = case
+    with tempfile.TemporaryDirectory() as tmp:
+        files = _fastq_pe(tmp, gs, G, n, L, seed) if layout[0] == "-p" else [_fastq(tmp, gs, G, n, L, seed, 0.002, 0.01)]
+        _engine_half(files, gs, layout)
+
+
 def _run_sorted(lib, case):
     gs, G, n, L, seed = case
     with tempfile.TemporaryDirectory() as tmp:
@@ -118,10 +179,11 @@ def test_live_host_paired_sorted_with_oracle_records(case):
     assert "segments" in _run_paired(_build_mock, case, order="s")
 
 
-@needs_bins
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", PAIRED_SORTED)
 def test_live_host_paired_sorted_on_gpu(case):
+    if not HAVE_BINS:
+        return _engine_half_of(case, ("-p", "-om", "s"))
     log = _run_paired(lambda tmp: REAL_LIB, case, order="s")
     assert "kernel launches" in log and " 0 kernel launches" not in log, log
 
@@ -133,18 +195,20 @@ def test_live_host_paired_multi_block_with_oracle_records():
     assert "segments" in _run_paired(_build_mock, (100, 400000, 35000, 150, 91))
 
 
-@needs_bins
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", SORTED)
 def test_live_host_sorted_on_gpu(case):
+    if not HAVE_BINS:
+        return _engine_half_of(case, ("-s", "-om", "s"))
     log = _run_sorted(lambda tmp: REAL_LIB, case)
     assert "kernel launches" in log and " 0 kernel launches" not in log, log
 
 
-@needs_bins
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", PAIRED)
 def test_live_host_paired_on_gpu(case):
+    if not HAVE_BINS:
+        return _engine_half_of(case, ("-p", "-om", "o"))
     log = _run_paired(lambda tmp: REAL_LIB, case)
     assert "kernel launches" in log and " 0 kernel launches" not in log, log
 
@@ -181,13 +245,14 @@ def test_live_host_ragged_reads_with_oracle_records(lo):
         assert "segments" in _check(_build_mock(tmp), 1, tmp, fq)
 
 
-@needs_bins
 @pytest.mark.gpu
 @pytest.mark.parametrize("lo", [25, 3])
 def test_live_host_ragged_reads_on_gpu(lo):
     with tempfile.TemporaryDirectory() as tmp:
         fq = _fastq(tmp, 1, 6000, 3000, 100, 77, 0.003, 0.01)
         _make_ragged(fq, 5, lo)
+        if not HAVE_BINS:
+            return _engine_half([fq], 1)
         log = _check(REAL_LIB, 1, tmp, fq)
         assert "kernel launches" in log and " 0 kernel launches" not in log, log
 
@@ -227,10 +292,24 @@ def test_live_host_default_kmer_lengths_with_oracle_records(name):
         assert "segments" in _run_golden_fqs(_build_mock(tmp), name, tmp)
 
 
-@pytest.mark.skipif(not os.path.exists(LIVE_BIN), reason="host/_bin not built")
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", ["se_orig_gs3100", "pe_orig_gs3100"])
 def test_live_host_default_kmer_lengths_on_gpu(name):
+    if not os.path.exists(LIVE_BIN):      # the engine half against the reference's own records, which ride in the fixture
+        g = H.load_golden(name)
+        pref, p, s, b = E.kmer_params(int(g["gs"]))
+        paired = "-p" in [str(x) for x in g["extra"]]
+        e = E.KmerEngine(p, s, b, pref, mode=E.MODE_PE_ORIGINAL if paired else E.MODE_SE_ORIGINAL)
+        if paired:
+            recs, info = H.run_pe(e, g["fastq"], is_gpu=True)
+            want, winfo = H.golden_pe_expect(g)
+            assert np.array_equal(info, winfo)
+        else:
+            recs, want = H.run_se(e, g["fastq"]), g["recs"][g["recs"]["pos"] < 0xFFFFFFF0]
+        H.assert_recs_equal(recs, want)
+        H.assert_dump_equal(e, g, pairs=paired)
+        e.close()
+        return
     with tempfile.TemporaryDirectory() as tmp:
         log = _run_golden_fqs(REAL_LIB, name, tmp)
         assert "kernel launches" in log and " 0 kernel launches" not in log, log
@@ -250,7 +329,6 @@ def test_live_host_fails_loudly_without_engine():
         assert r.returncode == 3 and "no CPU fallback" in r.stderr
 
 
-@needs_bins
 @pytest.mark.gpu
 @pytest.mark.parametrize("layout,case", [(("-s", "-om", "o"), CASES[0]), (("-p", "-om", "o"), PAIRED[0])])
 def test_live_host_count_records_on_gpu(layout, case, monkeypatch):
@@ -259,6 +337,10 @@ def test_live_host_count_records_on_gpu(layout, case, monkeypatch):
     covered on the GPU as well.  Both must give the reference's bytes."""
     monkeypatch.setenv("FQSK_CTX", "0")
     with tempfile.TemporaryDirectory() as tmp:
+        if not HAVE_BINS:      # the 28-byte count records through fqsk_submit / fqsk_collect
+            gs, G, n, L, seed = case[:5]
+            files = _fastq_pe(tmp, gs, G, n, L, seed) if layout[0] == "-p" else [_fastq(tmp, *case)]
+            return _engine_half(files, gs, layout, submit=True)
         if layout[0] == "-p":
             gs, G, n, L, seed = case
             log = _check(REAL_LIB, gs, tmp, _fastq_pe(tmp, gs, G, n, L, seed), layout=layout)
@@ -267,13 +349,14 @@ def test_live_host_count_records_on_gpu(layout, case, monkeypatch):
         assert "28-byte count records" in log, log
 
 
-@needs_bins
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", CASES + [BIG])
 def test_live_host_on_gpu(case):
     assert os.path.exists(REAL_LIB), "fqsqueezer_b200/libfqsk.so is not built"
     with tempfile.TemporaryDirectory() as tmp:
         fq = _fastq(tmp, *case)
+        if not HAVE_BINS:      # over several reads_blocks too (BIG), through fqsk_submit / fqsk_collect
+            return _engine_half([fq], case[0], submit=True)
         log = _check(REAL_LIB, case[0], tmp, fq, decode=case is not BIG)
         assert "kernel launches" in log and " 0 kernel launches" not in log, log
         assert "16-byte context records built on the device" in log, log

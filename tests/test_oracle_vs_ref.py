@@ -1,12 +1,80 @@
 """Unit-level pinning of the CPU oracle against the reference's own classes (oracle/_ref/libfqs_ref.so, a harness TU
-over kmer.h / ht_kmer.h / bit_vec.h / utils.h compiled from /root/reference by oracle/build_ref.py).
-Skipped where that library is absent."""
+over kmer.h / ht_kmer.h / bit_vec.h / utils.h compiled from the reference's sources by oracle/build_ref.py).
+
+The reference side `ru` of every test is checked against tests/golden/oracle_vs_ref_units.json: the SHA-256 of every output the
+reference side returned, call by call, for these seeded inputs.  Where the harness library is built, `ru` is the reference itself:
+its outputs must match the stored ones and the oracle must match it.  Where it is absent (a checkout holds only the repository), `ru`
+is a fresh oracle whose every output must match the stored reference output.  `source` in the file says which side recorded it:
+    FQS_RECORD_UNIT_DIGESTS=1 python -m pytest tests/test_oracle_vs_ref.py
+records from the reference where the harness is built, else from the oracle."""
+import hashlib
+import json
+import os
+
 import numpy as np
 import pytest
 
 from oracle import oracle as O
 
-pytestmark = pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref/libfqs_ref.so not built")
+DIGESTS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "oracle_vs_ref_units.json")
+RECORD = os.environ.get("FQS_RECORD_UNIT_DIGESTS") == "1"
+_recorded = {}
+
+
+def _digest(v):
+    if isinstance(v, tuple):
+        return [_digest(x)[0] for x in v]
+    a = np.ascontiguousarray(v)
+    return [hashlib.sha256(f"{a.dtype.str}{a.shape}".encode() + a.tobytes()).hexdigest()[:32]]
+
+
+class _Pinned:
+    """The reference side of one test: every call goes to `units` and its output is compared with (or, recording, appended to) the
+    stored digests of the reference's outputs, in call order.  Calls without an output (free, insert, clear) are not recorded."""
+
+    def __init__(self, units, calls, record):
+        self.units, self.calls, self.record, self.at, self.failed = units, calls, record, 0, False
+
+    def __getattr__(self, name):
+        fn = getattr(self.units, name)
+
+        def call(*args):
+            out = fn(*args)
+            if out is None or name.endswith("_new"):
+                return out
+            d = [name, _digest(out)]
+            if self.record:
+                self.calls.append(d)
+            else:
+                self.failed = self.at >= len(self.calls) or self.calls[self.at] != d
+                assert self.at < len(self.calls), f"call {self.at} ({name}): no stored reference output"
+                assert self.calls[self.at] == d, f"call {self.at} ({name}): differs from the reference's stored output"
+            self.at += 1
+            return out
+        return call
+
+
+@pytest.fixture(scope="module")
+def _stored():
+    if RECORD:
+        yield _recorded
+        src = "reference (oracle/_ref/libfqs_ref.so)" if O.have_ref() else "oracle (oracle/fqs_oracle.cpp)"
+        with open(DIGESTS, "w") as f:      # one line per test
+            f.write('{"source": %s,\n "calls": {\n' % json.dumps(src) +
+                    ",\n".join(f"  {json.dumps(k)}: {json.dumps(v)}" for k, v in sorted(_recorded.items())) + "\n}}\n")
+        return
+    with open(DIGESTS) as f:
+        yield json.load(f)["calls"]
+
+
+@pytest.fixture
+def ru(request, _stored):
+    units = O.ref_units() if O.have_ref() else O.oracle_units()
+    if RECORD:
+        _stored[request.node.name] = []
+    r = _Pinned(units, _stored.get(request.node.name, []), RECORD)
+    yield r
+    assert RECORD or r.failed or r.at == len(r.calls), f"{r.at} reference outputs seen, {len(r.calls)} stored"
 
 
 def _rand_regs(rng, k, n, cur=None):
@@ -26,9 +94,9 @@ def _normalize(d, rc, k):
     return np.where((d & km) < (rc & km), d, rc)
 
 
-def test_mt19937_stream():
+def test_mt19937_stream(ru):
     a = O.oracle_units().mt_stream(5481, 5000)
-    b = O.ref_units().mt_stream(5481, 5000)
+    b = ru.mt_stream(5481, 5000)
     assert np.array_equal(a, b)
     # known answers of the standard: default seed 5489 -> first output 3499211612, 10000th output 4123659995
     k = O.oracle_units().mt_stream(5489, 10000)
@@ -36,9 +104,9 @@ def test_mt19937_stream():
 
 
 @pytest.mark.parametrize("thr,mult,top", [(7, 2, 63), (2047, 1, 4095), (3, 1, 15)])
-def test_counter_incrementer(thr, mult, top):
+def test_counter_incrementer(thr, mult, top, ru):
     rng = np.random.default_rng(1)
-    ou, ru = O.oracle_units(), O.ref_units()
+    ou = O.oracle_units()
     co, cr = ou.cinc_new(thr, mult, top), ru.cinc_new(thr, mult, top)
     cnt = rng.integers(0, top + 1, 20000).astype(np.uint32)
     inc = rng.integers(0, top + 1, 20000).astype(np.uint32)
@@ -49,7 +117,7 @@ def test_counter_incrementer(thr, mult, top):
 
 
 @pytest.mark.parametrize("k", [14, 17, 19, 24, 27])
-def test_kmer_register_script(k):
+def test_kmer_register_script(k, ru):
     rng = np.random.default_rng(k)
     ops = [(0, 0, 0)]
     cur = 0
@@ -71,7 +139,7 @@ def test_kmer_register_script(k):
             ops.append((3, int(rng.integers(0, 4)), 0))
     ops = np.array(ops, np.uint32)
     a64, a32 = O.oracle_units().kmer_script(k, ops)
-    b64, b32 = O.ref_units().kmer_script(k, ops)
+    b64, b32 = ru.kmer_script(k, ops)
     full = b32[:, 2] == 1
     # dir / rc / aligned are defined for every state; normalised / kernel only compared on full registers
     assert np.array_equal(a64[:, [0, 1, 3, 4]], b64[:, [0, 1, 3, 4]])
@@ -80,9 +148,9 @@ def test_kmer_register_script(k):
 
 
 @pytest.mark.parametrize("k,cbits,item_bytes", [(19, 6, 4), (24, 6, 4), (27, 6, 4), (20, 12, 4), (24, 6, 8), (17, 12, 8)])
-def test_table_insert_find_count(k, cbits, item_bytes):
+def test_table_insert_find_count(k, cbits, item_bytes, ru):
     rng = np.random.default_rng(100 + k)
-    ou, ru = O.oracle_units(), O.ref_units()
+    ou = O.oracle_units()
     thr, mult, top = (7, 2, 63) if cbits == 6 else (2047, 1, 4095)
     to, tr = ou.ht_new(k, cbits), ru.ht_new(k, cbits, item_bytes)
     co, cr = ou.cinc_new(thr, mult, top), ru.cinc_new(thr, mult, top)
@@ -113,10 +181,10 @@ def test_table_insert_find_count(k, cbits, item_bytes):
 
 
 @pytest.mark.parametrize("k,missing", [(19, 1), (19, 2), (24, 3), (17, 4)])
-def test_table_find_partial(k, missing):
+def test_table_find_partial(k, missing, ru):
     """Front-truncated lookups: 4^m completions merged with PRNG-aware addition (ht_kmer.h:266-327)."""
     rng = np.random.default_rng(7 * k + missing)
-    ou, ru = O.oracle_units(), O.ref_units()
+    ou = O.oracle_units()
     to, tr = ou.ht_new(k, 6), ru.ht_new(k, 6, 4)
     co, cr = ou.cinc_new(7, 2, 63), ru.cinc_new(7, 2, 63)
     # universe: a few suffixes shared by many fronts so that several completions hit
@@ -151,9 +219,9 @@ def test_table_find_partial(k, missing):
     assert np.array_equal(ou.cinc_inc1(co, probe), ru.cinc_inc1(cr, probe))
 
 
-def test_small_int_vector():
+def test_small_int_vector(ru):
     rng = np.random.default_rng(5)
-    ou, ru = O.oracle_units(), O.ref_units()
+    ou = O.oracle_units()
     bits = 24
     so, sr = ou.siv_new(bits), ru.siv_new(bits)
     idx = rng.integers(0, 1 << bits, 300000).astype(np.uint64)
@@ -169,9 +237,9 @@ def test_small_int_vector():
                               ru.siv_test_shorter(sr, pre, np.full(len(pre), size, np.uint32)))
 
 
-def test_pair_table():
+def test_pair_table(ru):
     rng = np.random.default_rng(9)
-    ou, ru = O.oracle_units(), O.ref_units()
+    ou = O.oracle_units()
     k = 24
     po, pr = ou.pair_new(k), ru.pair_new(k, 1)
     vm = (1 << (2 * k)) - 1
