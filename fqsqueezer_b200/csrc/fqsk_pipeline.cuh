@@ -1233,12 +1233,6 @@ __device__ __forceinline__ void block_scan_chunk(T (&v)[NQ][ITEMS], T (&ex)[NQ][
 	__syncthreads();
 }
 
-struct SegTotals {        // written by the scan kernels, read by the host once per segment
-	unsigned long long n_rec; U64x4 letters;
-	uint32_t tot_b, tot_s, tot_p, hidden;
-	unsigned long long draws_b, draws_s;
-};
-
 // Scans over per-read arrays, one CTA per chunk of 1024 * ITEMS reads (a single CTA is bound by what one SM can pull from
 // HBM: 0.28 ms for 51 000 reads).  Every CTA scans its chunk, publishes the chunk totals tagged with the launch epoch and adds
 // up the totals of the CTAs before it (cta_chain_prefix).  Grids are small (<= 2 CTAs per SM), so all CTAs are co-resident and
@@ -1475,19 +1469,19 @@ __global__ void __launch_bounds__(256) k_ctx_codes(EngineDev E, SegDev S, PipeDe
 	out[g] = fqsk_ctx_make(rec.counts, rec.level, rec.rough, rec.cor_pos, i, pos, read_len, sym, n_run, r_hist, s64, E.p, E.s, E.b);
 }
 
-// the host's look at the device: status block (128 words) + counters (6 x u64) into the page-locked look buffer, then -- after a
-// system-wide fence -- the sequence number the host is spinning on
-__global__ void __launch_bounds__(160) k_publish(const uint32_t *status, const unsigned long long *counters, uint32_t *out, unsigned long long *seq, unsigned long long want) { pdl_enter();
-	const uint32_t t = threadIdx.x;
-	if (t < 128) out[t] = status[t];
-	else if (t < 134) reinterpret_cast<unsigned long long *>(out + 128)[t - 128] = counters[t - 128];
+// the host's look at the device: the status block into its page-locked mirror, then -- after a system-wide fence -- the sequence
+// number the host is spinning on
+__global__ void __launch_bounds__(128) k_publish(const EngineStatus *status, EngineStatus *out, unsigned long long *seq, unsigned long long want) { pdl_enter();
+	const uint32_t *src = reinterpret_cast<const uint32_t *>(status);
+	uint32_t *dst = reinterpret_cast<uint32_t *>(out);
+	for (uint32_t i = threadIdx.x; i < sizeof(EngineStatus) / 4; i += blockDim.x) dst[i] = src[i];
 	__threadfence_system();
 	__syncthreads();
-	if (t == 0) { *reinterpret_cast<volatile unsigned long long *>(seq) = want; __threadfence_system(); }
+	if (threadIdx.x == 0) { *reinterpret_cast<volatile unsigned long long *>(seq) = want; __threadfence_system(); }
 }
 // a segment evaluated again (retry): the reset k_prep did for the first evaluation
-__global__ void k_seg_reset(uint8_t *status, unsigned long long *counters) { pdl_enter();
-	seg_reset_words(status, counters, threadIdx.x);
+__global__ void k_seg_reset(EngineStatus *status) { pdl_enter();
+	seg_reset_words(status, threadIdx.x);
 }
 // Verdict of a segment's first pass for the sync that is enqueued behind it without a host look + the state the next segment
 // inherits (read_prev, dna.cpp:1550-1551; in sorted order pmer_can_prev, dna.cpp:655), in one launch.  The pass settled when no
